@@ -35,11 +35,21 @@ PRESETS = {
 }
 
 
+DUMP_BYTES = 64 * 10**6      # --dump-outputs: at most this many bytes of .npy files in all
+
+
+def _positive(s):
+    n = int(s)
+    if n < 1:
+        raise argparse.ArgumentTypeError(f"must be >= 1, got {n}")
+    return n
+
+
 def parse(argv=None):
     argv = list(sys.argv[1:] if argv is None else argv)
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=_positive, default=5, help="timed steps (each timed loop runs exactly this many)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--mode", default=os.environ.get("LCA_BENCH_MODE", "fwdbwd"), choices=["fwd", "fwdbwd"])
@@ -67,7 +77,14 @@ def parse(argv=None):
     ap.add_argument("--configs", default="", help="comma-separated BASELINE config ids: run them all in ONE process group "
                     "(one JSON line per config x mode; saves the spawn + NCCL bootstrap of separate launches)")
     ap.add_argument("--modes", default="", help="with --configs: comma-separated modes (fwd,fwdbwd); default --mode")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned to its caller (out; dq, dk, dv "
+                         "in fwdbwd mode) as DIR/<name>.npy in float32, stacked over ranks; a seeded sample of token "
+                         "rows when the whole would exceed 64 MB.  The inputs depend only on the arguments, so two "
+                         "builds can be compared output for output")
     a = ap.parse_args(argv)
+    if a.dump_outputs and a.configs:
+        ap.error("--dump-outputs writes one configuration; it cannot be combined with --configs")
     if a.config:
         given = {x.split("=")[0].lstrip("-").replace("-", "_") for x in argv if x.startswith("--")}
         for key, val in PRESETS[a.config].items():
@@ -150,6 +167,33 @@ class _HostCuda:
     @staticmethod
     def set_device(i):
         pass
+
+
+def dump_outputs(path, arrays, dist, rank, budget=DUMP_BYTES):
+    """Writes every (B, S/N, H, D) shard of ``arrays`` (name -> tensor) as ``path/<name>.npy``: float32, shape
+    (N, B, rows, H, D), rank r's shard at index r.  ``dist`` is None in a single process.  When all shards of all
+    arrays exceed ``budget`` bytes, the same seeded sample of local token rows (sorted) is taken from each of them.
+    Every rank must call this; rank 0 writes.  Returns a description of what was written."""
+    import numpy as np
+    import torch
+
+    world = dist.get_world_size() if dist is not None else 1
+    Sl = next(iter(arrays.values())).shape[1]
+    row_bytes = 4 * world * sum(t[:, 0].numel() for t in arrays.values())
+    n = min(Sl, (budget - 1024 * len(arrays)) // row_bytes)          # 1 KiB per file covers the .npy header
+    rows = torch.arange(Sl) if n == Sl else torch.randperm(Sl, generator=torch.Generator().manual_seed(0))[:n].sort().values
+    if rank == 0:
+        os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        s = t.detach()[:, rows.to(t.device)].float().contiguous()
+        parts = [s]
+        if dist is not None:
+            parts = [torch.empty_like(s) for _ in range(world)]
+            dist.all_gather(parts, s)
+        if rank == 0:
+            np.save(os.path.join(path, name + ".npy"), torch.stack(parts).cpu().numpy())
+    return {"dir": path, "arrays": list(arrays), "dtype": "float32", "layout": "(rank, batch, row, head, dim)",
+            "rows_per_rank": int(n), "local_seq": int(Sl), "row_sample_seed": None if n == Sl else 0}
 
 
 def main():
@@ -263,7 +307,7 @@ def run_config(a, ctx):
 
     def to_dev(non_blocking=True):
         """This step's inputs: q, k, v (and the upstream gradient dO in fwd+bwd mode) from pinned host memory."""
-        ts = [t.to(dev, non_blocking=non_blocking) for t in host]
+        ts = [t.to(dev, non_blocking=non_blocking, copy=True) for t in host]     # copy: fresh leaves on cpu too
         if need_grad:
             ts = [t.requires_grad_() for t in ts]
             ts.append(host_do.to(dev, non_blocking=non_blocking))
@@ -327,6 +371,7 @@ def run_config(a, ctx):
     results = []
 
     def run_pipelined(n):
+        """Returns the last step's inputs and output."""
         nxt = prefetch()
         for i in range(n):
             ts, ev = nxt
@@ -338,13 +383,14 @@ def run_config(a, ctx):
                 nxt = prefetch()          # H2D of step i+1 overlaps the attention of step i
             out = step(*ts)
             results.append(float(out.float().mean().item()))     # D2H read of the step's result
+        return ts, out
 
     run_pipelined(3)        # warm the pipelined path with the same allocation pattern (two input sets in flight)
     cu.synchronize(dev)
     barrier()
     t_ev0, t_ev1 = cu.Event(enable_timing=True), cu.Event(enable_timing=True)
     t_ev0.record()
-    run_pipelined(a.steps)
+    last_in, last_out = run_pipelined(a.steps)
     t_ev1.record()
     barrier()
     clocks = sampler.stop()
@@ -354,6 +400,16 @@ def run_config(a, ctx):
         t = torch.tensor([ms, ms_e2e], device=dev, dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms, ms_e2e = float(t[0]), float(t[1])
+
+    # The last timed step takes fresh leaf tensors from the same host inputs as every other step, so its gradients
+    # are that step's alone (the device-resident loop accumulates into q/k/v.grad across steps).
+    dumped = None
+    if a.dump_outputs:
+        arrays = {"out": last_out}
+        if need_grad:
+            arrays.update(dq=last_in[0].grad, dk=last_in[1].grad, dv=last_in[2].grad)
+        dumped = dump_outputs(a.dump_outputs, arrays, dist if world > 1 else None, rank)
+    del last_in, last_out
 
     # ------------------------------------------------------------------ exposed communication (ours, N > 1)
     # The same tcgen05 kernels on the same per-rank problem (this rank's ring block of queries against all S keys,
@@ -501,6 +557,7 @@ def run_config(a, ctx):
             "config_id": a.config or 3,
             "check": check,
             "staging": staging,
+            "outputs": dumped,
         }))
     del attn
     if a.impl == "ours" and check is not None and not check.get("ok", False):

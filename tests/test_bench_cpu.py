@@ -39,6 +39,53 @@ def test_bench_single_process_contract():
     assert e["d2h_bytes_per_step"] == 4 and d["ms_per_step"] > 0 and e["ms_per_step"] > 0
 
 
+def test_bench_dump_outputs_repeat_exactly(tmp_path):
+    """``--dump-outputs``: out / dq / dk / dv of the last timed step as float32, identical for identical inputs (the
+    gradients are that step's alone, whatever the number of steps)."""
+    import numpy as np
+    dumps = []
+    for run, steps in (("a", "2"), ("b", "3")):
+        d = _run(1, 0, "--steps", steps, "--dump-outputs", str(tmp_path / run))
+        assert d["steps"] == int(steps)
+        assert d["outputs"]["arrays"] == ["out", "dq", "dk", "dv"] and d["outputs"]["rows_per_rank"] == 256
+        dumps.append({n: np.load(tmp_path / run / f"{n}.npy") for n in d["outputs"]["arrays"]})
+    for n, x in dumps[0].items():
+        assert x.dtype == np.float32 and x.shape == (1, 1, 256, 4, 16) and np.isfinite(x).all()
+        assert np.array_equal(x, dumps[1][n]), n
+    assert np.abs(dumps[0]["dq"]).max() > 0
+
+
+def test_bench_dump_outputs_two_ranks_forward(tmp_path):
+    d = _run(2, 29861, "--mode", "fwd", "--dump-outputs", str(tmp_path))
+    import numpy as np
+    out = np.load(tmp_path / "out.npy")
+    assert d["outputs"]["arrays"] == ["out"] and out.shape == (2, 1, 128, 4, 16) and out.dtype == np.float32
+    assert sorted(os.listdir(tmp_path)) == ["out.npy"]
+
+
+def test_dump_outputs_samples_rows_within_budget(tmp_path):
+    import importlib.util
+
+    import numpy as np
+    import torch
+    spec = importlib.util.spec_from_file_location("bench", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    x = torch.randn(2, 1000, 3, 8, dtype=torch.bfloat16)
+    y = torch.randn(2, 1000, 1, 8)
+    budget = 40_000
+    info = bench.dump_outputs(str(tmp_path), {"x": x, "y": y}, None, 0, budget=budget)
+    n = info["rows_per_rank"]
+    assert 0 < n < 1000 and info["row_sample_seed"] == 0
+    assert sum(os.path.getsize(tmp_path / f) for f in os.listdir(tmp_path)) <= budget
+    xs, ys = np.load(tmp_path / "x.npy"), np.load(tmp_path / "y.npy")
+    assert xs.shape == (1, 2, n, 3, 8) and ys.shape == (1, 2, n, 1, 8)
+    rows = torch.randperm(1000, generator=torch.Generator().manual_seed(0))[:n].sort().values
+    assert np.array_equal(xs[0], x[:, rows].float().numpy()) and np.array_equal(ys[0], y[:, rows].numpy())
+    again = bench.dump_outputs(str(tmp_path / "again"), {"x": x, "y": y}, None, 0, budget=budget)
+    assert again == {**info, "dir": str(tmp_path / "again")}
+
+
 @pytest.mark.parametrize("flags", [
     (),
     ("--mode", "fwd", "--ring-impl", "strip"),
